@@ -1,19 +1,25 @@
 #!/usr/bin/env python
 """bench.py -- agent-steps/sec of the DecentralPlannerNet hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" = one addGSO + forward of one batch of synthetic rollout-like input at the configuration
 BASELINE.json quotes the metric on (configs[1], "C2"): DCP K=3, 10 agents, 20x20 map, batch 64
 inference per GPU (640 agent-steps per step per GPU, weak scaling, no collective on the data path).
 
-How every number is timed: W untimed warm-up steps, then R windows of EXACTLY K back-to-back steps, each
-window bracketed by CUDA events on the launching stream; R is chosen so that the windows cover >= ~100 ms
-(a single 20-step window is 1.2 ms here -- shorter than a host scheduler quantum, which made the 8-rank
-maximum a measure of submission jitter in round 1).  A rank's figure is the MEDIAN window, the reported
-figure the MAX over ranks of that, after a barrier + torch.cuda.synchronize() on both sides.  Inputs rotate
-through a device pool larger than L2.
+How every number is timed: untimed warm-up steps (at least W and at least half a second, so that clocks, the
+library's lanes and the host loop are in steady state), then exactly K back-to-back timed steps, after a barrier +
+torch.cuda.synchronize() on both sides.  CUDA events on the launching stream (wall clock for the host calls) split the
+K steps into up to 10 consecutive windows; a rank's figure is K times the MEDIAN per-step time of its windows (robust to
+host scheduler hiccups, which a single window of a host-bound loop is not), the reported figure the MAX over ranks.  The
+default K = 5000 makes the headline window about 110 ms on a B200 (22.4 us per step measured at a 1000 W power limit);
+much shorter windows measure host submission jitter more than the GPU.  The legs time their own step counts derived
+from K (below).  Inputs rotate through a device pool larger than L2.
+
+--dump-outputs DIR   after the timed steps, writes the logits [10 agents, 64 episodes, 5 actions] (float32) that the
+        last timed step of `value` returned to DIR/logits.npy (rank 0).  The inputs depend only on the arguments, so two
+        builds run with the same arguments can be compared output for output.
 
 value   C2 device-resident (inputs already in HBM), 6 independent episode batches in flight over the library's compute
         lanes (DecentralPlannerNet.infer_async / join); `single_stream` = the same steps one after the other on one stream.
@@ -77,7 +83,8 @@ def config_dict(world):
     return {"workload": WORKLOAD, "K": K_TAPS, "num_agents": N_AGENTS, "map_w": MAP_W, "batch_per_gpu": BATCH,
             "global_batch": BATCH * world,
             "parallelism": "episode-sharded replicas x%d, no collective on the inference data path" % world,
-            "timing": "median of R windows of K steps (CUDA events), R windows >= ~100 ms, max over ranks",
+            "timing": "K timed steps after >= W warm-up steps and >= 0.5 s, in up to 10 windows (CUDA events), median window, "
+                      "max over ranks",
             "l2_policy": "device-resident inputs rotate through a pool > 126 MB L2"}
 
 
@@ -253,74 +260,85 @@ def time_cpu(step, budget_s, min_steps=5, warmup=3):
 
 
 # ----------------------------------------------------------------------------------------------------------
-# timing helper: R windows of K steps
+# timing helper: K steps in up to WINDOWS consecutive windows
 # ----------------------------------------------------------------------------------------------------------
 class Timer:
-    def __init__(self, dist, dev, target_ms=100.0, max_windows=400):
-        self.dist, self.dev, self.target_ms, self.max_windows = dist, dev, target_ms, max_windows
+    WINDOWS = 10
+    SETTLE_S = 0.5
+
+    def __init__(self, dist, dev):
+        self.dist, self.dev = dist, dev
+
+    def _bounds(self, K):
+        n = min(K, self.WINDOWS)
+        return [round(j * K / n) for j in range(n + 1)]
+
+    def _warm_up(self, step, warmup, drain, period):
+        """Untimed steps 0 .. n-1: `warmup` of them, then more in rounds of `warmup` until every rank has spent at least
+        SETTLE_S seconds, then up to n = warmup modulo `period` so that the timed steps n, n+1, ... see the same inputs
+        however long the warm-up took.  Whether to run another round is decided over all ranks, so every rank runs the
+        same n steps: a step may contain a collective (the training legs' gradient all-reduce).  Returns n."""
+        self.barrier()
+        t0, n, rnd = time.perf_counter(), 0, max(1, warmup)
+        while True:
+            for _ in range(rnd):
+                step(n)
+                n += 1
+            (more,) = self.max_over_ranks(float(time.perf_counter() - t0 < self.SETTLE_S))
+            if not more:
+                break
+        while (n - warmup) % period:
+            step(n)
+            n += 1
+        drain()
+        self.barrier()
+        return n
+
+    @staticmethod
+    def _median_ms(K, bounds, ms):
+        """K x the median per-step ms of the windows; ms[w] is window w's duration."""
+        return K * float(np.median([ms[w] / (bounds[w + 1] - bounds[w]) for w in range(len(ms))]))
 
     def barrier(self):
         if self.dist is not None:
             self.dist.barrier()
         torch.cuda.synchronize()
 
-    def device_windows(self, step, K, warmup, drain=None):
-        """step(i) enqueues one step on the current stream (or on the library's lanes: then drain() makes the current
-        stream wait for everything outstanding before a window's closing event).  Returns (median window ms on this
-        rank, windows)."""
+    def device_window(self, step, K, warmup, drain=None, period=1):
+        """step(i) enqueues one step on the current stream (or on the library's lanes, whose steps the current stream
+        joins as it goes: then drain() makes it wait for everything outstanding before the last window's closing event).
+        After the warm-up (_warm_up) the next K steps are timed.  Returns K x the median per-step ms of the windows on
+        this rank."""
         drain = drain or (lambda: None)
-        for i in range(warmup):
-            step(i)
-        drain()
-        torch.cuda.synchronize()
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record()
-        for i in range(K):
-            step(warmup + i)
-        drain()
-        e1.record()
-        torch.cuda.synchronize()
-        probe = max(e0.elapsed_time(e1), 1e-3)
-        R = int(min(self.max_windows, max(3, round(self.target_ms / probe))))
-        self.barrier()
-        evs = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(R)]
-        n = warmup + K
-        for a, b in evs:
-            a.record()
-            for i in range(K):
+        n = self._warm_up(step, warmup, drain, period)
+        bounds = self._bounds(K)
+        evs = [torch.cuda.Event(enable_timing=True) for _ in bounds]
+        evs[0].record()
+        for w in range(len(bounds) - 1):
+            for i in range(bounds[w], bounds[w + 1]):
                 step(n + i)
-            drain()
-            b.record()
-            n += K
+            if w == len(bounds) - 2:
+                drain()
+            evs[w + 1].record()
         torch.cuda.synchronize()
         self.barrier()
-        return float(np.median([a.elapsed_time(b) for a, b in evs])), R
+        return self._median_ms(K, bounds, [evs[w].elapsed_time(evs[w + 1]) for w in range(len(bounds) - 1)])
 
-    def host_windows(self, step, K, warmup, drain):
-        """step(i) is a host call (may leave work in flight; drain() completes it).  Wall-clock windows."""
-        for i in range(warmup):
-            step(i)
-        drain()
-        torch.cuda.synchronize()
-        t0 = time.perf_counter()
-        for i in range(K):
-            step(warmup + i)
-        drain()
-        torch.cuda.synchronize()
-        probe = max((time.perf_counter() - t0) * 1e3, 1e-3)
-        R = int(min(self.max_windows, max(3, round(self.target_ms / probe))))
-        self.barrier()
-        times, n = [], warmup + K
-        for _ in range(R):
-            t0 = time.perf_counter()
-            for i in range(K):
+    def host_window(self, step, K, warmup, drain):
+        """step(i) is a host call (may leave work in flight; drain() completes it before the last window closes).
+        Wall-clock windows, warm-up and result as in device_window."""
+        n = self._warm_up(step, warmup, drain, 1)
+        bounds = self._bounds(K)
+        ts = [time.perf_counter()]
+        for w in range(len(bounds) - 1):
+            for i in range(bounds[w], bounds[w + 1]):
                 step(n + i)
-            drain()
-            torch.cuda.synchronize()
-            times.append((time.perf_counter() - t0) * 1e3)
-            n += K
+            if w == len(bounds) - 2:
+                drain()
+                torch.cuda.synchronize()
+            ts.append(time.perf_counter())
         self.barrier()
-        return float(np.median(times)), R
+        return self._median_ms(K, bounds, [(ts[w + 1] - ts[w]) * 1e3 for w in range(len(bounds) - 1)])
 
     def max_over_ranks(self, *vals):
         if self.dist is None:
@@ -453,10 +471,10 @@ def leg_inference(gp, timer, dev, rank, world, n, k, batch, map_w, gso_dtype, K,
         model.addGSO(pool_S[i % pool_n])
         return model(pool_x[i % pool_n])
     with torch.no_grad():
-        ms, R = timer.device_windows(step, K, warmup)
+        ms = timer.device_window(step, K, warmup)
     (ms,) = timer.max_over_ranks(ms)
     out = {"workload": label, "ms_per_step": ms / K, "us_per_step": 1e3 * ms / K,
-           "agent_steps_per_s": world * batch * n * K / (ms * 1e-3), "windows": R, "gso_dtype": str(np.dtype(gso_dtype))}
+           "agent_steps_per_s": world * batch * n * K / (ms * 1e-3), "steps": K, "gso_dtype": str(np.dtype(gso_dtype))}
     if global_batch is not None:
         out["scaling"] = "strong"
         out["global_batch"] = batch * world
@@ -473,7 +491,7 @@ def leg_inference(gp, timer, dev, rank, world, n, k, batch, map_w, gso_dtype, K,
         # the rollout step as the reference's agent runs it: host tensors in, logits out, one blocking call
         hx, hS = [t.pin_memory() for t in xs_h], [t.pin_memory() for t in Ss_h]
         hout = torch.empty(n, batch, 5).pin_memory()
-        hms, hR = timer.host_windows(lambda i: model.infer_host(hx[i % 4], hS[i % 4], hout), K, warmup, lambda: None)
+        hms = timer.host_window(lambda i: model.infer_host(hx[i % 4], hS[i % 4], hout), K, warmup, lambda: None)
         (hms,) = timer.max_over_ranks(hms)
         out["host_call_us_per_step"] = 1e3 * hms / K
         out["host_call_api"] = "DecentralPlannerNet.infer_host (pinned host x / float64 S in, logits out, blocking)"
@@ -509,10 +527,10 @@ def leg_rollout(gp, timer, dev, rank, world, n, k, episodes, map_w, K, warmup, l
         l0 = _lib.launch_count()
         step(1)
         launches = _lib.launch_count() - l0
-        ms, R = timer.device_windows(step, K, warmup)
+        ms = timer.device_window(step, K, warmup)
     (ms,) = timer.max_over_ranks(ms)
     out = {"workload": label, "us_per_step": 1e3 * ms / K, "episode_steps_per_s": world * episodes * K / (ms * 1e-3),
-           "agent_steps_per_s": world * episodes * n * K / (ms * 1e-3), "windows": R, "launches_per_step": int(launches),
+           "agent_steps_per_s": world * episodes * n * K / (ms * 1e-3), "steps": K, "launches_per_step": int(launches),
            "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
     if cpu:
         from oracle import sim_oracle
@@ -559,9 +577,9 @@ def leg_training(gp, timer, dist, dev, rank, world, n, batch, map_w, K, warmup, 
     step(0)
     torch.cuda.synchronize()
     launches = _lib.launch_count()
-    ms, R = timer.device_windows(step, K, warmup)
+    ms = timer.device_window(step, K, warmup)
     (ms,) = timer.max_over_ranks(ms)
-    out = {"workload": label, "ms_per_step": ms / K, "agent_steps_per_s": world * batch * n * K / (ms * 1e-3), "windows": R,
+    out = {"workload": label, "ms_per_step": ms / K, "agent_steps_per_s": world * batch * n * K / (ms * 1e-3), "steps": K,
            "library_launches_per_step": int(launches),
            "step": "train-mode forward + fused loss (gpp_planner_ce_loss) + backward + %sAdam"
                    % ("one flat 826 KB gradient all-reduce (NCCL, inside the timed step) + " if world > 1 else "")}
@@ -637,7 +655,10 @@ def main():
     ap.add_argument("--sat-batch", type=int, default=131072,
                     help="episodes in the saturated graph-filter roofline measurement (0 = skip)")
     ap.add_argument("--no-legs", action="store_true", help="headline configuration only")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's logits to DIR/logits.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -648,7 +669,7 @@ def main():
         args.warmup = args.warmup if args.warmup is not None else 3
         run_reference(args, rank, world)
         return
-    args.steps = args.steps if args.steps is not None else 200
+    args.steps = args.steps if args.steps is not None else 5000
     args.warmup = max(3, args.warmup if args.warmup is not None else 20)
     K, W = args.steps, args.warmup
 
@@ -682,16 +703,17 @@ def main():
             dev_step(i)
         torch.cuda.synchronize()
         launches_per_window = _lib.launch_count()      # library kernels in one K-step window
-        single_ms, single_R = timer.device_windows(dev_step, K, W)      # one stream, one batch after the other
+        single_ms = timer.device_window(dev_step, K, W)      # one stream, one batch after the other
         # the same steps as a driver of independent episode batches issues them: DEV_DEPTH batches in flight over the
         # library's compute lanes (DecentralPlannerNet.infer_async / join), device tensors in, device logits out; the
         # closing event of a window waits for every outstanding step
         DEV_DEPTH = 6
         dev_outs = [torch.empty(N_AGENTS, BATCH, 5, device=dev) for _ in range(DEV_DEPTH)]
-        dev_inflight = []
+        dev_inflight, dev_last = [], [0]
 
         def dev_async_step(i):
             tk, _ = model.infer_async(pool_x[i % pool_n], pool_S[i % pool_n], dev_outs[i % DEV_DEPTH])
+            dev_last[0] = i % DEV_DEPTH
             dev_inflight.append(tk)
             if len(dev_inflight) >= DEV_DEPTH:
                 model.join(dev_inflight.pop(0))
@@ -699,7 +721,10 @@ def main():
         def dev_drain():
             while dev_inflight:
                 model.join(dev_inflight.pop(0))
-        ms, R = timer.device_windows(dev_async_step, K, W, dev_drain)
+        ms = timer.device_window(dev_async_step, K, W, dev_drain, period=pool_n)
+        if args.dump_outputs and rank == 0:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            np.save(os.path.join(args.dump_outputs, "logits.npy"), dev_outs[dev_last[0]].cpu().numpy())
 
         # ---- per-kernel durations (events recorded around each kernel; PDL is off in this pass) -------
         nat = model._native_for(dev)
@@ -717,8 +742,8 @@ def main():
         hS = [t.pin_memory() for t in Ss_h]
         hout = torch.empty(N_AGENTS, BATCH, 5).pin_memory()
         # (a) one blocking host call per step
-        sync_ms, sync_R = timer.host_windows(lambda i: model.infer_host(hx[i % unique], hS[i % unique], hout), K, W,
-                                             lambda: None)
+        sync_ms = timer.host_window(lambda i: model.infer_host(hx[i % unique], hS[i % unique], hout), K, W,
+                                    lambda: None)
         # (b) pipelined over independent episode batches: step i is enqueued before step i - (DEPTH - 1) is waited for, as
         # a rollout driver advancing DEPTH groups of episodes in turn would do; every step still reads its x / S from
         # pinned host memory and writes its logits back to it.  The library rotates the tickets over 4 compute lanes.
@@ -738,10 +763,10 @@ def main():
                     tk, slot = inflight.pop(0)
                     model.wait(tk)
                     sink[0] += float(houts[slot][0, 0, 0])
-            return timer.host_windows(async_step, K, W, drain)
+            return timer.host_window(async_step, K, W, drain)
         DEPTH = 6
-        e2e_ms, e2e_R = pipelined(DEPTH)
-        e2e3_ms, _ = pipelined(3)
+        e2e_ms = pipelined(DEPTH)
+        e2e3_ms = pipelined(3)
     ms, e2e_ms, sync_ms, e2e3_ms, single_ms = timer.max_over_ranks(ms, e2e_ms, sync_ms, e2e3_ms, single_ms)
     clocks = sampler.summary()
 
@@ -783,20 +808,17 @@ def main():
         gf_gbs = gf_bytes_per_agent_step(N_AGENTS) * agent_steps / gf_s / 1e9
         sm_mhz = clocks.get("sm_mhz") or clocks.get("sm_max_mhz") or 1965.0
         fp32_peak = 148 * 128 * 2 * float(sm_mhz) * 1e6 / 1e12
-        cfg = config_dict(world)
-        cfg["windows"] = R
         line = {
             "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": K,
             "warmup": W, "ms_per_step": ms / K, "higher_is_better": True,
             "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
-            "config": cfg,
+            "config": config_dict(world),
             "value_api": "DecentralPlannerNet.infer_async / join -> gpp_planner_forward_async: device tensors in, device logits "
                          "out, %d independent episode batches in flight over the library's 4 compute lanes" % DEV_DEPTH,
             "single_stream": {"value": world * agent_steps * K / (single_ms * 1e-3), "ms_per_step": single_ms / K,
-                              "windows": single_R,
                               "api": "model.addGSO(S); model(x) on one stream, one batch after the other (the latency "
                                      "of a step; kernels chained by programmatic dependent launch)"},
-            "e2e": {"value": world * agent_steps * K / (e2e_ms * 1e-3), "unit": UNIT, "steps": K, "windows": e2e_R,
+            "e2e": {"value": world * agent_steps * K / (e2e_ms * 1e-3), "unit": UNIT, "steps": K,
                     "h2d_bytes_per_step": bytes_per_batch, "d2h_bytes_per_step": N_AGENTS * BATCH * 5 * 4,
                     "api": "DecentralPlannerNet.infer_host_async/wait -> gpp_planner_forward_host_async (pinned host "
                            "buffers; inputs staged by the copy engine on a copy stream, forward on one of four compute "
@@ -804,9 +826,9 @@ def main():
                            "idle, logits written straight to host), %d independent episode batches in flight" % DEPTH,
                     "batches_in_flight": DEPTH,
                     "value_3_in_flight": world * agent_steps * K / (e2e3_ms * 1e-3),
-                    "sync_value": world * agent_steps * K / (sync_ms * 1e-3), "sync_windows": sync_R,
+                    "sync_value": world * agent_steps * K / (sync_ms * 1e-3),
                     "sync_api": "DecentralPlannerNet.infer_host -> gpp_planner_forward_host, one blocking call per step"},
-            "gpu_launches": int(launches_per_window) * R, "gpu_launches_per_step": int(launches_per_window) / K,
+            "gpu_launches": int(launches_per_window), "gpu_launches_per_step": int(launches_per_window) / K,
             "clocks": clocks,
             "roofline": {"kernel": "feature_mma_kernel (per-agent CNN + compress MLP on tcgen05: fp16 2-way split operands, "
                                    "3 products per term, fp32 accumulation in TMEM -- the dominant kernel of the step by time)",

@@ -1,9 +1,8 @@
-"""TEST INFRASTRUCTURE ONLY -- import the *unmodified* reference from /root/reference.
+"""TEST INFRASTRUCTURE ONLY -- import the *unmodified* reference from its checkout (REF_ROOT below).
 
-Only usable inside the build container (the GPU box has no /root/reference).
-Used by tests/golden/make_golden.py to generate the committed golden vectors and
-by the container-only tests that pin oracle/planner_oracle.py against the real
-reference code.  Nothing here is imported by the product package.
+Only usable where that checkout exists.  Used by tests/golden/make_golden.py and
+tests/golden/make_reference_checks.py to generate the committed golden vectors that
+pin oracle/planner_oracle.py.  Nothing here is imported by the product package.
 
 Why a shim is needed (SURVEY.md section 8c):
   * /root/reference/utils/__init__.py and graphs/__init__.py eagerly import every

@@ -1,5 +1,6 @@
 """TEST INFRASTRUCTURE ONLY -- drive the reference's own rollout simulator (utils/multirobotsim_dcenlocal.py, unmodified,
-from /root/reference) step by step with given logits.  Build container only.  `random.choice` (:490) is replaced by the
+from its checkout, oracle/ref_agent.py) step by step with given logits; reference_rollout needs that checkout,
+oracle_rollout (the same rollout through oracle/sim_oracle.py) does not.  `random.choice` (:490) is replaced by the
 round-robin contract of oracle/sim_oracle.py for the duration of a rollout, so that the reference becomes deterministic."""
 from __future__ import annotations
 
