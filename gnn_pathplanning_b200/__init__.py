@@ -14,8 +14,9 @@ from .graphml import (BatchLSIGF, GraphFilterBatch, GraphFilterL2ShareBatch, Gra
                       graph_filter, torchpermul, FEATURE_MAJOR, NODE_MAJOR)
 from .planner import DecentralPlannerNet, planner_loss, weights_init
 from .rollout import BatchedRollout
+from .evaluation import CaseRecords, summarize
 
-__all__ = ["DecentralPlannerNet", "GraphFilterBatch", "BatchLSIGF", "graph_filter", "weights_init", "planner_loss", "BatchedRollout", "GraphFilterRNNBatch", "GraphFilterMoRNNBatch", "GraphFilterL2ShareBatch", "torchpermul",
+__all__ = ["DecentralPlannerNet", "GraphFilterBatch", "BatchLSIGF", "graph_filter", "weights_init", "planner_loss", "BatchedRollout", "CaseRecords", "summarize", "GraphFilterRNNBatch", "GraphFilterMoRNNBatch", "GraphFilterL2ShareBatch", "torchpermul",
            "FEATURE_MAJOR", "NODE_MAJOR", "install_dropin", "build"]
 
 

@@ -101,6 +101,64 @@ def make_batch(batch: int, num_agents: int, map_w: int, seed: int = 1337,
     return x, S.astype(gso_dtype)
 
 
+_MOVES = ((-1, 0), (0, -1), (1, 0), (0, 1))   # up, left, down, right (multirobotsim_dcenlocal.py:21-25); 4 = stop
+
+
+def _bfs_distance(map_hw: np.ndarray, goal) -> np.ndarray:
+    """Steps from every free cell to `goal` over free cells (4-connected); -1 = unreachable."""
+    W = map_hw.shape[0]
+    dist = np.full(map_hw.shape, -1, dtype=np.int64)
+    dist[goal[0], goal[1]] = 0
+    frontier = [(int(goal[0]), int(goal[1]))]
+    while frontier:
+        nxt = []
+        for x, y in frontier:
+            for dx, dy in _MOVES:
+                u, v = x + dx, y + dy
+                if 0 <= u < W and 0 <= v < W and map_hw[u, v] == 0 and dist[u, v] < 0:
+                    dist[u, v] = dist[x, y] + 1
+                    nxt.append((u, v))
+        frontier = nxt
+    return dist
+
+
+def random_eval_cases(rng: np.random.Generator, batch: int, num_agents: int, map_w: int, density: float = 0.1):
+    """B test cases in the test loader's content: maps [B,W,W] int64, starts / goals [B,N,2] int64 with no agent
+    starting on its goal, one-hot expert actions [B,N,T,5] float32 and makespan [B] int64.  The expert is each agent's
+    own shortest path (breadth-first search; the first shortest move in action order), ignoring the other agents --
+    enough for the target makespan / flowtime the test loop replays.  makespan = the longest of a case's paths;
+    T = the longest over the batch, shorter paths are padded with 'stop'."""
+    maps, starts, goals, paths = [], [], [], []
+    while len(maps) < batch:
+        m, st, gl = random_episode(rng, num_agents, map_w, density)
+        if (st == gl).all(axis=1).any():
+            continue
+        acts = []
+        for s, g in zip(st, gl):
+            dist = _bfs_distance(m, g)
+            if dist[s[0], s[1]] < 0:
+                break
+            x, y, a = int(s[0]), int(s[1]), []
+            while dist[x, y] > 0:
+                k = next(k for k, (dx, dy) in enumerate(_MOVES)
+                         if 0 <= x + dx < map_w and 0 <= y + dy < map_w and dist[x + dx, y + dy] == dist[x, y] - 1)
+                a.append(k)
+                x, y = x + _MOVES[k][0], y + _MOVES[k][1]
+            acts.append(a)
+        if len(acts) < num_agents:
+            continue                                  # some goal unreachable: draw the case again
+        maps.append(m); starts.append(st); goals.append(gl); paths.append(acts)
+    makespan = np.array([max(len(a) for a in p) for p in paths], dtype=np.int64)
+    T = int(makespan.max())
+    target = np.zeros((batch, num_agents, T, 5), dtype=np.float32)
+    target[..., 4] = 1.0
+    for b, p in enumerate(paths):
+        for i, a in enumerate(p):
+            target[b, i, np.arange(len(a)), 4] = 0.0
+            target[b, i, np.arange(len(a)), a] = 1.0
+    return np.stack(maps), np.stack(starts), np.stack(goals), target, makespan
+
+
 def random_targets(batch: int, num_agents: int, seed: int = 1337) -> np.ndarray:
     """Uniform random one-hot action targets [B,N,5] (int64), the training label
     format of Dataloader_dcplocal_notTF_onlineExpert.py:142-157."""

@@ -223,6 +223,37 @@ int gpp_rollout_move(const float* logits, int* pos, const int* goal, const unsig
                      int* last_action, unsigned int* choice_counter, int* flags, int currentstep, int B, int N,
                      int W, void* stream);
 
+/* ------------------------------------------------------------------------------------
+ * Per-case evaluation of the lock-step rollout (replaces the bookkeeping of the reference's test() loop,
+ * agents/decentralplannerlocal.py:484-648, that surrounds the model and the simulator's move).  Device pointers,
+ * int32 unless stated.
+ *
+ * gpp_rollout_targets replays the expert's actions (multiRobotSim.getPathTarget, utils/multirobotsim_dcenlocal.py
+ * :159-229), one warp per case:
+ *   target  f32 [B,N,T,5] one-hot expert actions (the test loader's format); action = first maximum of each row
+ *   start, goal [B,N,2]
+ *   target_start / target_end out [B,N]: first step with a non-stop action / step + 1 of the first arrival (-1 = never)
+ *   targets out [B,3] = {makespanTarget = max(end) - min(start), flowtimeTarget = sum(end - start), every agent
+ *   arrived}; both metrics are 0 unless every agent arrived (an agent with start == goal counts as not arrived).
+ *
+ * gpp_rollout_track runs once per step after gpp_rollout_move, with the same flags / active / maxstep: for every case
+ * with active[b] != 0 it ORs check_moveCollision and check_predictCollsion into status[b] (:593-598), stores the move's
+ * allReachGoal and currentstep, and clears active[b] when allReachGoal || currentstep >= maxstep[b] (:600-606).
+ *   status [B,4] in/out = {allReachGoal of the last move, collision happened in the loop, collision predicted in the
+ *   loop, step of the last move}; zero it before the first step.
+ *
+ * gpp_rollout_evaluate_finish runs once after the loop, one warp per case, and writes what mutliAgent_ActionPolicy
+ * returns (:611-624, with checkOptimality :825-832 and the predicted metrics of move :693-715):
+ *   record out [B,10] = {allReachGoal, noReachGoalbyCollsionShielding, findOptimalSolution, check_collisionFreeSol,
+ *   check_CollisionPredictedinLoop, makespanPredict, makespanTarget, flowtimePredict, flowtimeTarget,
+ *   num_agents_reachgoal}, from status, targets, maxstep and gpp_rollout_move's reached / start_step / end_step. */
+int gpp_rollout_targets(const float* target, const int* start, const int* goal, int* target_start, int* target_end,
+                        int* targets, int B, int N, int T, void* stream);
+int gpp_rollout_track(const int* flags, int* active, int* status, const int* maxstep, int currentstep, int B,
+                      void* stream);
+int gpp_rollout_evaluate_finish(const int* status, const int* targets, const int* maxstep, const int* reached,
+                                const int* start_step, const int* end_step, int* record, int B, int N, void* stream);
+
 /* Asynchronous variant for pipelined rollouts over INDEPENDENT episode batches: stages the inputs on a copy stream,
  * enqueues the forward on one of the planner's four compute streams (tickets rotate over them, so the feature kernel of
  * one batch runs next to the kernels of the batches before it on the SMs they leave idle) and returns at once with a completion ticket; the
