@@ -15,8 +15,9 @@ from .graphml import (BatchLSIGF, GraphFilterBatch, GraphFilterL2ShareBatch, Gra
 from .planner import DecentralPlannerNet, planner_loss, weights_init
 from .rollout import BatchedRollout
 from .evaluation import CaseRecords, summarize
+from .dataset import ExpertDataset, read_ecbs_solutions, read_mat_cases, write_failure_cases
 
-__all__ = ["DecentralPlannerNet", "GraphFilterBatch", "BatchLSIGF", "graph_filter", "weights_init", "planner_loss", "BatchedRollout", "CaseRecords", "summarize", "GraphFilterRNNBatch", "GraphFilterMoRNNBatch", "GraphFilterL2ShareBatch", "torchpermul",
+__all__ = ["DecentralPlannerNet", "GraphFilterBatch", "BatchLSIGF", "graph_filter", "weights_init", "planner_loss", "BatchedRollout", "CaseRecords", "summarize", "ExpertDataset", "read_ecbs_solutions", "read_mat_cases", "write_failure_cases", "GraphFilterRNNBatch", "GraphFilterMoRNNBatch", "GraphFilterL2ShareBatch", "torchpermul",
            "FEATURE_MAJOR", "NODE_MAJOR", "install_dropin", "build"]
 
 

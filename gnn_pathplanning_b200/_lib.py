@@ -14,8 +14,8 @@ import threading
 PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 CSRC_DIR = os.path.join(PKG_DIR, "csrc")
 LIB_PATH = os.path.join(PKG_DIR, "libgnnpp_b200.so")
-SOURCES = ("graph_filter.cu", "graph_filter_tc.cu", "graph_filter_pair.cu", "graph_filter_small.cu", "rollout.cu", "evaluate.cu", "feature.cu", "feature_tc.cu", "feature_mma.cu", "train.cu", "planner.cu")
-HEADERS = ("common.cuh", "feature.cuh", "tc_common.cuh")
+SOURCES = ("graph_filter.cu", "graph_filter_tc.cu", "graph_filter_pair.cu", "graph_filter_small.cu", "rollout.cu", "evaluate.cu", "dataset.cu", "feature.cu", "feature_tc.cu", "feature_mma.cu", "train.cu", "planner.cu")
+HEADERS = ("common.cuh", "feature.cuh", "tc_common.cuh", "step_inputs.cuh")
 INCLUDE = os.path.join(os.path.dirname(PKG_DIR), "include", "gnnpp_b200.h")
 INCLUDE_DEBUG = os.path.join(os.path.dirname(PKG_DIR), "include", "gnnpp_b200_debug.h")
 
@@ -39,6 +39,7 @@ EXPORTED = (
     "gpp_planner_forward", "gpp_planner_forward_host",
     "gpp_planner_train_workspace_bytes", "gpp_planner_train_forward", "gpp_planner_train_backward", "gpp_planner_ce_loss", "gpp_rollout_build_inputs", "gpp_rollout_move",
     "gpp_rollout_targets", "gpp_rollout_track", "gpp_rollout_evaluate_finish",
+    "gpp_dataset_prepare", "gpp_dataset_batch",
     "gpp_planner_forward_host_async", "gpp_planner_wait", "gpp_planner_forward_async", "gpp_planner_join",
     "gpp_planner_set_profiling", "gpp_planner_get_profile",
     "gpp_planner_set_graph_filter_mode", "gpp_planner_set_feature_mode",
@@ -188,6 +189,10 @@ def load():
         lib.gpp_rollout_track.argtypes = [vp, vp, vp, vp, i, i, vp]
         lib.gpp_rollout_evaluate_finish.restype = i
         lib.gpp_rollout_evaluate_finish.argtypes = [vp, vp, vp, vp, vp, vp, vp, i, i, vp]
+        lib.gpp_dataset_prepare.restype = i
+        lib.gpp_dataset_prepare.argtypes = [vp, vp, C.c_double, vp, i, i, vp]
+        lib.gpp_dataset_batch.restype = i
+        lib.gpp_dataset_batch.argtypes = [vp, vp, vp, vp, vp, i, vp, vp, vp, vp, vp, i, i, i, i, vp]
         lib.gpp_planner_forward_host_async.restype = i
         lib.gpp_planner_forward_host_async.argtypes = [vp, vp, vp, i, vp, i, i, C.POINTER(C.c_ulonglong)]
         lib.gpp_planner_wait.restype = i

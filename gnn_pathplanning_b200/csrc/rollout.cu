@@ -10,15 +10,9 @@
 // integer agent positions that never leave the device; rollout_move_kernel turns the planner's logits into moves with the
 // reference's edge / obstacle / inter-robot collision shielding.  Both are integer / IEEE-double restatements of the
 // reference's arithmetic: bit-exact by construction (tests/test_gpu_rollout.py).
-#include "common.cuh"
+#include "step_inputs.cuh"
 
 namespace gpp {
-
-constexpr int RO_MAX_N = 64;        // agents per episode (one 64-bit adjacency mask per agent)
-constexpr int RO_FOV = 9;           // statetransformer.py:11
-constexpr int RO_HALF = 4;          // :12  FOV_width
-constexpr int RO_WIN = 11;          // :14-15  FOV + 2 * border
-constexpr int RO_CENTER = 5;        // :16,20-21
 
 struct RoInputArgs {
     const int* pos;        // [B][N][2] current agent cells (x, y)
@@ -59,31 +53,9 @@ __global__ void __launch_bounds__(128) rollout_inputs_kernel(const RoInputArgs a
     for (int guard = 0; guard < 4096; ++guard) {
         if (tid == 0 && a.grow_radius) rad = rad * 1.1;
         __syncthreads();
-        if (tid < N) {
-            unsigned long long m = 0ull;
-            const double r = rad;
-            for (int j = 0; j < N; ++j) {
-                const int dx = px[tid] - px[j], dy = py[tid] - py[j];
-                const double d = sqrt((double)(dx * dx + dy * dy));        // scipy pdist (euclidean, float64)
-                if (j != tid && d < r) m |= 1ull << j;
-            }
-            adj[tid] = m;
-        }
+        if (tid < N) adj[tid] = ro_adjacency_row(tid, N, px, py, rad);
         __syncthreads();
-        if (tid == 0) {
-            // isConnected (graphTools.py:396-423) counts zero eigenvalues of the Laplacian = connected components;
-            // the same predicate by breadth-first search over the adjacency masks
-            unsigned long long seen = 1ull, frontier = 1ull;
-            while (frontier) {
-                unsigned long long nxt = 0ull;
-                for (int i = 0; i < N; ++i)
-                    if (frontier >> i & 1ull) nxt |= adj[i];
-                frontier = nxt & ~seen;
-                seen |= nxt;
-            }
-            const unsigned long long all = N >= 64 ? ~0ull : ((1ull << N) - 1ull);
-            is_conn = (seen & all) == all;
-        }
+        if (tid == 0) is_conn = ro_is_connected(adj, N);
         __syncthreads();
         if (!a.grow_radius || is_conn) break;
     }
@@ -92,50 +64,17 @@ __global__ void __launch_bounds__(128) rollout_inputs_kernel(const RoInputArgs a
         if (a.connected) a.connected[b] = is_conn;
     }
     // ---- D^-1/2 A D^-1/2 with the zero-degree guard (:341-348), float64 as the reference
-    if (tid < N) {
-        const int deg = __popcll(adj[tid]);
-        dinv[tid] = deg ? sqrt(1.0 / (double)deg) : 0.0;
-    }
+    if (tid < N) dinv[tid] = ro_deg_inv_sqrt(adj[tid]);
     __syncthreads();
     for (int e = tid; e < N * N; e += blockDim.x) {
         const int i = e / N, j = e - i * N;
-        const double v = (adj[i] >> j & 1ull) ? dinv[i] * dinv[j] : 0.0;       // (Deg @ A) @ Deg with A in {0, 1}
+        const double v = ro_gso_entry(adj, dinv, i, j);
         if (a.s_is_f64) reinterpret_cast<double*>(a.S)[(size_t)b * N * N + e] = v;
         else reinterpret_cast<float*>(a.S)[(size_t)b * N * N + e] = (float)v;
     }
-    // ---- field-of-view tensor (statetransformer.py:82-130): channel 0 obstacle window (outside the map = obstacle),
-    //      channel 1 goal (inside the 9x9 view, else projected onto the rim of the 11x11 window, :47-66), channel 2 agents
-    float* xo = a.x + (size_t)b * N * 3 * RO_WIN * RO_WIN;
-    for (int e = tid; e < N * 3 * RO_WIN * RO_WIN; e += blockDim.x) {
-        const int i = e / (3 * RO_WIN * RO_WIN), rem = e - i * 3 * RO_WIN * RO_WIN;
-        const int ch = rem / (RO_WIN * RO_WIN), uv = rem - ch * RO_WIN * RO_WIN, u = uv / RO_WIN, v = uv - u * RO_WIN;
-        const int cx = px[i], cy = py[i];
-        float val = 0.f;
-        if (ch != 1) {
-            if (u >= 1 && u <= RO_FOV && v >= 1 && v <= RO_FOV) {
-                const int gx = cx - RO_HALF + (u - 1), gy = cy - RO_HALF + (v - 1);
-                const bool inside = gx >= 0 && gx < W && gy >= 0 && gy < W;
-                if (ch == 0) val = inside ? (map[gx * W + gy] ? 1.f : 0.f) : 1.f;
-                else val = inside && (occ_bits[(gx * W + gy) >> 5] >> ((gx * W + gy) & 31) & 1u) ? 1.f : 0.f;
-            }
-        } else {
-            const int dx = goal[2 * i] - cx, dy = goal[2 * i + 1] - cy;
-            int tx, ty;
-            if (abs(dx) <= RO_HALF && abs(dy) <= RO_HALF) {
-                tx = RO_CENTER + dx;
-                ty = RO_CENTER + dy;
-            } else if (dy != 0 && abs(dx) <= abs(dy)) {
-                // bearing within [pi/4, 3pi/4] or [-3pi/4, -pi/4] (:56): |dx| <= |dy|; np.round = round half to even
-                ty = RO_CENTER * ((dy > 0) - (dy < 0) + 1);
-                tx = RO_CENTER + (int)rint((double)RO_CENTER * (double)dx / (double)abs(dy));
-            } else {
-                tx = RO_CENTER * ((dx > 0) - (dx < 0) + 1);
-                ty = RO_CENTER + (int)rint((double)RO_CENTER * (double)dy / (double)abs(dx));
-            }
-            val = (u == tx && v == ty) ? 1.f : 0.f;
-        }
-        xo[e] = val;
-    }
+    // ---- field-of-view tensor (statetransformer.py:82-130)
+    float* xo = a.x + (size_t)b * N * RO_FOV_ELEMS;
+    for (int e = tid; e < N * RO_FOV_ELEMS; e += blockDim.x) xo[e] = ro_fov_value(e, px, py, goal, map, occ_bits, W);
 }
 
 struct RoMoveArgs {

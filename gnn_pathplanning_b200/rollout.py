@@ -10,8 +10,9 @@ host <-> device copy -- only the `done` flags are read back every `poll_every` s
 Mirrors the simulator's interface where it has one: `setup`, `getCurrentState`, `getGSO`, `move`, `getMaxstep`,
 `count_numAgents_ReachGoal`, plus `run(model)` for the whole loop.  `setup_cases` + `evaluate(model)` replace the
 reference's test() loop (agents/decentralplannerlocal.py:484-648): per-case success / makespan / flowtime records,
-summarised by `evaluation.summarize`.  The only behavioural difference is the documented tie-break contract of
-gpp_rollout_move (round-robin instead of `random.choice`).
+summarised by `evaluation.summarize`; `failure_cases()` lists the cases the online expert would re-plan.  The only
+behavioural difference is the documented tie-break contract of gpp_rollout_move (round-robin instead of
+`random.choice`).
 """
 from __future__ import annotations
 
@@ -189,6 +190,15 @@ class BatchedRollout:
                 self.start_step.data_ptr(), self.end_step.data_ptr(), record.data_ptr(), self.B, self.N,
                 self._stream()))
         return CaseRecords.from_record(record.cpu().numpy(), self.N)
+
+    def failure_cases(self):
+        """After evaluate(): the cases whose loop ended at maxstep (currentStep >= maxstep, a success on the last step
+        included) -- the ones the reference's online expert hands to its solver (agents/
+        decentralplannerlocal_OnlineExpert.py:536-539).  Returns (case indices [F] int64, the agents' final cells
+        [F,N,2] int64) on the host, for `dataset.write_failure_cases`."""
+        assert self.targets is not None and self.step > 0, "failure_cases() needs a finished evaluate()"
+        ids = torch.nonzero(self.status[:, 3] >= self.maxstep).reshape(-1)
+        return ids.cpu().numpy(), self.pos[ids].long().cpu().numpy()
 
 
 _DELTA = np.array([[-1, 0], [0, -1], [1, 0], [0, 1], [0, 0]], dtype=np.int64)    # multirobotsim_dcenlocal.py:21-25

@@ -165,3 +165,32 @@ def random_targets(batch: int, num_agents: int, seed: int = 1337) -> np.ndarray:
     rng = np.random.default_rng(seed + 1)
     idx = rng.integers(0, 5, size=(batch, num_agents))
     return np.eye(5, dtype=np.int64)[idx]
+
+
+def random_schedules(rng: np.random.Generator, cases: int, num_agents: int, map_w: int, density: float = 0.1,
+                     max_len: int = 31, p_wait: float = 0.2):
+    """Expert-schedule-like cases for `ExpertDataset.add`: per case [T_c,N,2] int64 cells, goals [C,N,2] int64 and maps
+    [C,W,W] int64.  Each agent walks from a distinct free cell for 1 .. max_len - 1 moves (random free neighbour, or a
+    wait with probability p_wait or when boxed in) and then stays; its goal is its last cell and T_c is the case's
+    longest walk + 1 -- the rows a solver's schedule turns into.  Agents may share cells: the transformer never checks."""
+    C, N, W = cases, num_agents, map_w
+    maps = (rng.random((C, W, W)) < density).astype(np.int64)
+    pos = np.empty((C, N, 2), dtype=np.int64)
+    for c in range(C):
+        free = np.flatnonzero(maps[c] == 0)
+        cell = rng.choice(free, N, replace=False)
+        pos[c, :, 0], pos[c, :, 1] = cell // W, cell % W
+    length = rng.integers(1, max_len, size=(C, N))                 # moves per agent
+    traj = [pos.copy()]
+    ci = np.arange(C)[:, None]
+    for t in range(max_len - 1):
+        k = rng.integers(0, 4, size=(C, N))
+        nxt = pos + np.asarray(_MOVES)[k]
+        inside = ((nxt >= 0) & (nxt < W)).all(-1)
+        ok = inside & (maps[ci, nxt[..., 0].clip(0, W - 1), nxt[..., 1].clip(0, W - 1)] == 0)
+        ok &= (rng.random((C, N)) >= p_wait) & (t < length)
+        pos = np.where(ok[..., None], nxt, pos)
+        traj.append(pos.copy())
+    traj = np.stack(traj, axis=1)                                   # [C,max_len,N,2]
+    T = length.max(axis=1) + 1
+    return [traj[c, :T[c]] for c in range(C)], traj[np.arange(C), T - 1], maps

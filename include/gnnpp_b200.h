@@ -254,6 +254,31 @@ int gpp_rollout_track(const int* flags, int* active, int* status, const int* max
 int gpp_rollout_evaluate_finish(const int* status, const int* targets, const int* maxstep, const int* reached,
                                 const int* start_step, const int* end_step, int* record, int B, int N, void* stream);
 
+/* ------------------------------------------------------------------------------------
+ * Training samples from expert schedules (replaces the online expert's DataTransformer, onlineExpert/
+ * DataTransformer_local_onlineExpert.py:96-305, and the train loader's per-sample scipy.io.loadmat,
+ * dataloader/Dataloader_dcplocal_notTF_onlineExpert.py:142-157).  Device pointers, int32 unless stated.  C cases
+ * stored as one flat row array: case c has T_c = makespan + 1 rows case_first_row[c] .. case_first_row[c+1] - 1 of
+ *   pos  [R,N,2] agent cells per step, R = sum of T_c (row t of a case: the expert's cell at step t, the goal after its
+ *        plan ends)
+ *
+ * gpp_dataset_prepare computes each case's communication threshold as computeAdjacencyMatrix(states, r0) does: start
+ * at r0, multiply by 1.1 (float64) while a step is disconnected, never reset between steps; the final value is used
+ * for every step.  case_first_row [C+1] (absolute row indices into pos); radius out f64 [C].  One CTA per case.
+ *
+ * gpp_dataset_batch builds B training samples in one launch, one CTA per sample:
+ *   row_case [R]; goal [C,N,2]; map [C,W,W] or (map_shared) [W,W] uint8, 1 = obstacle; radius [C] from prepare;
+ *   rows int64 [B] sample (= row) indices, a row outside [0, R) gives an all-zero sample;
+ *   x out f32 [B,N,3,11,11] (toSeqInputTensor's field of view); S out f32 [B,N,N] (the float32 cast of the float64
+ *   D^-1/2 A D^-1/2 with A = pdist < radius, zero diagonal); target out int64 [B,N,5] one-hot index of the move to the
+ *   next row (to the goal on a case's last row) in delta = up, left, down, right, stop.
+ * Both support 2 <= N <= 64 and square maps with W*W <= 327,680 cells, else GPP_ERR_UNSUPPORTED. */
+int gpp_dataset_prepare(const int* pos, const int* case_first_row, double r0, double* radius, int C, int N,
+                        void* stream);
+int gpp_dataset_batch(const int* pos, const int* row_case, const int* case_first_row, const int* goal,
+                      const unsigned char* map, int map_shared, const double* radius, const long long* rows, float* x,
+                      float* S, long long* target, int B, int N, int W, int R, void* stream);
+
 /* Asynchronous variant for pipelined rollouts over INDEPENDENT episode batches: stages the inputs on a copy stream,
  * enqueues the forward on one of the planner's four compute streams (tickets rotate over them, so the feature kernel of
  * one batch runs next to the kernels of the batches before it on the SMs they leave idle) and returns at once with a completion ticket; the
